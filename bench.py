@@ -35,6 +35,13 @@ against the CPU oracle, before the timed region), at N = 1 a `configs` block
 them) and `cpu_baseline` (the oracle port on a planted row slab of the same
 width, every host thread; measured per-step time and scale factor are separate
 keys, `extrapolated` says so).
+
+--dump-outputs DIR writes what the last timed solve returned to its caller as
+DIR/<name>.npy (float64): the iterate `x` after K steps and the per-iteration
+records `gamma`, `norm_res`, `objective`.  The inputs are generated from a
+fixed seed, so two builds run with the same arguments can be compared output
+for output.  An array that would push the total past 64 MB is replaced by a
+fixed, seeded sample of its entries.
 """
 import argparse
 import json
@@ -265,6 +272,21 @@ def run_reference(args):
 # ----------------------------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------------------------
+DUMP_BUDGET_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy in float64; an array over its share of DUMP_BUDGET_BYTES is replaced by the
+    entries at a fixed, seeded, sorted sample of its indices (the same sample in every run with the same sizes)."""
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (DUMP_BUDGET_BYTES // len(arrays) - 128) // 8          # 128: the .npy header
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def dmma_peak():
     """fp64 tensor-pipe peak measured by tools/probes/fp64_peak_probe.cu on this pool's B200 (profiles/r02_fp64_peaks.jsonl)."""
     p = os.path.join(ROOT, "profiles", "r02_fp64_peaks.jsonl")
@@ -570,6 +592,9 @@ def run_b200(args):
     med = order[len(order) // 2]
     dev_ms, e2e_s, launches = samples[med]
     last = recs[K - 1]
+    if args.dump_outputs and rank == 0:                        # x is replicated on every rank; xo is reused by later solves
+        dump_outputs(args.dump_outputs, {"x": xo, "gamma": [r.gamma for r in recs], "norm_res": [r.norm_res for r in recs],
+                                         "objective": [r.f_x + r.g_x for r in recs]})
 
     # per-kernel-family timing (profile breakdown; the shares the ncu launch list must agree with)
     ms_n = max_over_ranks(P["A"].time_kernel(0, reps=3))
@@ -688,7 +713,13 @@ def main():
     ap.add_argument("--nccl", action="store_true", help="A/B (N > 1): ncclAllReduce per iteration instead of the in-kernel all-reduce")
     ap.add_argument("--cpu-steps", type=int, default=20)
     ap.add_argument("--cpu-rows", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write x and the per-iteration records of the last timed solve to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
     if args.two_pass:
         os.environ["ADAPROX_FUSED"] = "0"
     if args.impl == "reference":
