@@ -799,15 +799,17 @@ def adaptive_proxgrad(x, *, f, g, rule, tol=1e-5, maxit=100_000, name="AdaPGM", 
 
 
 def adaptive_proxgrad_path(X0=None, *, f, lambdas, rule, gamma0=None, tol=1e-5, maxit=100_000, history=0):
-    """Batched multi-lambda lasso path (BASELINE config 5; include/adaprox.h: adaprox_solve_lambda_path): column j of the
+    """Batched multi-lambda path (BASELINE config 5; include/adaprox.h: adaprox_solve_lambda_path): column j of the
     result is what ``adaptive_proxgrad(X0[:, j], f=f, g=NormL1(lambdas[j]), rule=rule_j, tol=tol, maxit=maxit)`` returns,
-    where rule_j is ``rule`` with ``gamma = gamma0[j]`` when ``gamma0`` is given.  ``f`` must be a dense
-    ``LinearLeastSquares``.  Returns ``(X, its, info)`` with X of shape (n, L), ``its`` the per-column iteration counts
-    and ``info`` holding per-column ``norm_res``, ``gamma``, ``f_x`` and, with ``history = H > 0``, the arrays
-    ``gamma_hist``, ``res_hist``, ``obj_hist`` of shape (min(H, maxit), L) (NaN after a column stopped)."""
+    where rule_j is ``rule`` with ``gamma = gamma0[j]`` when ``gamma0`` is given.  ``f`` is a ``LinearLeastSquares`` over
+    a dense or scipy sparse matrix, or a ``LogisticLoss`` over a scipy sparse matrix; for the logistic loss n is
+    features + 1 (``LogisticLoss.n``, intercept last, penalised by the l1 term like every other entry).  Returns
+    ``(X, its, info)`` with X of shape (n, L), ``its`` the per-column iteration counts and ``info`` holding per-column
+    ``norm_res``, ``gamma``, ``f_x`` and, with ``history = H > 0``, the arrays ``gamma_hist``, ``res_hist``, ``obj_hist``
+    of shape (min(H, maxit), L) (NaN after a column stopped)."""
     ff, _ = _unwrap(f)
-    if not isinstance(ff, LinearLeastSquares):
-        raise L.AdaproxError(-3, "adaptive_proxgrad_path: f must be a LinearLeastSquares term (no CPU fallback)")
+    if not isinstance(ff, (LinearLeastSquares, LogisticLoss)):
+        raise L.AdaproxError(-3, "adaptive_proxgrad_path: f must be a LinearLeastSquares or LogisticLoss term (no CPU fallback)")
     lam = np.ascontiguousarray(np.asarray(lambdas, dtype=F64).ravel())
     Lc = lam.shape[0]
     n = ff.n if getattr(ff, "n", None) is not None else ff.A.shape[1]

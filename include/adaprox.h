@@ -221,14 +221,19 @@ int adaprox_logistic_grad_hessian(adaprox_handle h, adaprox_id X_mat, adaprox_id
 int adaprox_solve(adaprox_handle h, const adaprox_problem* p, const adaprox_options* o, const double* x0,
                   const double* y0, double* x_out, double* y_out, adaprox_record* records, adaprox_result* res);
 
-/* ---- batched multi-lambda lasso path (BASELINE config 5) --------------------- */
+/* ---- batched multi-lambda path (BASELINE config 5) ----------------------------- */
 /* AdaPGM (src/AdaProx.jl:418-421 -> :312-364 with A = 0, h = Zero) on the L problems
- *     min_x 1/2 |A x - b|^2 + lambdas[j] |x|_1 ,  j = 0 .. L-1
- * that share the dense least-squares term of `p` (lasso/runme.jl:16-27; p->g is ignored).  The reference has no batched
+ *     min_x f(x) + lambdas[j] |x|_1 ,  j = 0 .. L-1
+ * that share the smooth term f of `p` (p->g is ignored).  f is
+ *   - least squares 1/2 |A x - b|^2 (lasso/runme.jl:16-27) over a dense or a CSR matrix, or
+ *   - the logistic loss of sparse_logreg/runme.jl:18-39 over a CSR matrix (n = features + 1, intercept last and
+ *     penalised by the l1 term like every other entry).
+ * Dense logistic, a row-sharded matrix and other f kinds return ADAPROX_ERR_UNSUPPORTED.  The reference has no batched
  * entry point: running adaptive_proxgrad once per lambda is the behaviour this call reproduces column by column -- every
  * column has its own stepsize state, residual and stopping iteration and is frozen when it converges (its result is the
- * iterate the single-lambda call returns).  The L iterates advance together so that A*X and A'*R are fp64 tensor-core
- * contractions (mma.sync DMMA) instead of 2 L matrix-vector products.
+ * iterate the single-lambda call returns).  The L iterates advance together: for a dense matrix A*X and A'*R are fp64
+ * tensor-core contractions (mma.sync DMMA) instead of 2 L matrix-vector products; for a CSR matrix both sweeps gather whole
+ * lambda-contiguous rows of the iterate / residual block, so every gathered 32-byte sector is used.
  *   gamma0  : L initial stepsizes, or NULL to use o->gamma for every column
  *   x0T     : [L][n] (column j contiguous), or NULL for zeros
  *   x_outT  : [L][n];  iters / norm_res / gamma_out / f_out : [L] (each may be NULL)
