@@ -801,7 +801,8 @@ def adaptive_proxgrad(x, *, f, g, rule, tol=1e-5, maxit=100_000, name="AdaPGM", 
 def adaptive_proxgrad_path(X0=None, *, f, lambdas, rule, gamma0=None, tol=1e-5, maxit=100_000, history=0):
     """Batched multi-lambda path (BASELINE config 5; include/adaprox.h: adaprox_solve_lambda_path): column j of the
     result is what ``adaptive_proxgrad(X0[:, j], f=f, g=NormL1(lambdas[j]), rule=rule_j, tol=tol, maxit=maxit)`` returns,
-    where rule_j is ``rule`` with ``gamma = gamma0[j]`` when ``gamma0`` is given.  ``f`` is a ``LinearLeastSquares`` over
+    where rule_j is ``rule`` with ``gamma = gamma0[j]`` when ``gamma0`` is given (with ``FixedStepsize`` every step of column j
+    uses ``gamma0[j]``; ``maxit = 0`` returns the first prox step with ``its = 0``).  ``f`` is a ``LinearLeastSquares`` over
     a dense or scipy sparse matrix, or a ``LogisticLoss`` over a scipy sparse matrix; for the logistic loss n is
     features + 1 (``LogisticLoss.n``, intercept last, penalised by the l1 term like every other entry).  Returns
     ``(X, its, info)`` with X of shape (n, L), ``its`` the per-column iteration counts and ``info`` holding per-column

@@ -278,8 +278,9 @@ __global__ void __launch_bounds__(kCPFinWarps * 32) k_csr_path_finish(CsrPathArg
     } else {
       st.gamma = gamma; st.sigma = sigma; st.s0 = s0; st.s1 = s1; st.norm_res = norm_res; st.f_x = f_x;
       cs.gamma = gamma; cs.gl = gamma * st.lambda;
-      if (stop || (it >= a.O.maxit && it > 0)) {
-        // converged: the result is x_it (:355); maxit: the reference returns x after the last prox (:361-363)
+      if (stop || it >= a.O.maxit) {
+        // converged: the result is x_it (:355); maxit: the reference returns x after the last prox (:361-363), which at
+        // maxit = 0 is the prologue's x_1 (:330-332)
         st.it_done = it; st.flags = stop ? ADAPROX_FLAG_CONVERGED : 0u;
         cs.mode = stop ? CP_CONV : CP_MAXIT;
       } else {

@@ -364,8 +364,10 @@ __global__ void __launch_bounds__(kPT, 2) k_path_step(PathStepArgs a) {
       s_bc[threadIdx.x] = s;
     }
     __syncthreads();
+    DOpts Oc = a.O;
+    if (Oc.rule == ADAPROX_RULE_FIXED) Oc.gamma = gamma;                 // the column's own fixed stepsize (gamma0)
     const double gamma_prev = gamma;
-    rule_step(a.O, s_bc[1], s_bc[2], s_bc[3], gamma, sigma, s0, s1);     // :341
+    rule_step(Oc, s_bc[1], s_bc[2], s_bc[3], gamma, sigma, s0, s1);       // :341
     norm_res = sqrt(norm_sq_jl(s_bc[0]) + adapgm_dual_res_sq(gamma, gamma_prev, sigma));   // :348 (dual part: 0, or NaN -- phases.cuh)
     if (norm_res <= a.O.tol) stop = true;                                // :354
   }
@@ -387,8 +389,9 @@ __global__ void __launch_bounds__(kPT, 2) k_path_step(PathStepArgs a) {
     }
   }
   if (frozen) return;
-  if (stop || (it >= a.O.maxit && it > 0)) {
-    // converged: the result is x_it (:355); maxit: the reference returns x after the last prox (:361-363)
+  if (stop || it >= a.O.maxit) {
+    // converged: the result is x_it (:355); maxit: the reference returns x after the last prox (:361-363), which at
+    // maxit = 0 is the prologue's x_1 = prox(x_0 - gamma_0 grad f(x_0)) (:330-332)
     const bool conv = stop;
     if (conv) {
       for (int64_t q = threadIdx.x; q < a.n; q += kPT) a.XoutT[j * a.ldx + q] = x[q];

@@ -234,7 +234,9 @@ int adaprox_solve(adaprox_handle h, const adaprox_problem* p, const adaprox_opti
  * iterate the single-lambda call returns).  The L iterates advance together: for a dense matrix A*X and A'*R are fp64
  * tensor-core contractions (mma.sync DMMA) instead of 2 L matrix-vector products; for a CSR matrix both sweeps gather whole
  * lambda-contiguous rows of the iterate / residual block, so every gathered 32-byte sector is used.
- *   gamma0  : L initial stepsizes, or NULL to use o->gamma for every column
+ *   gamma0  : L initial stepsizes, or NULL to use o->gamma for every column; with FixedStepsize column j keeps
+ *             gamma0[j] for every step.  maxit = 0 returns x_1 = prox(x_0 - gamma_0 grad f(x_0)) with iters 0, as
+ *             adaptive_proxgrad does
  *   x0T     : [L][n] (column j contiguous), or NULL for zeros
  *   x_outT  : [L][n];  iters / norm_res / gamma_out / f_out : [L] (each may be NULL)
  *   hist    : optional 3 * hist_rows * L doubles: gamma, norm_res, objective per (iteration - 1, column); NaN where a
