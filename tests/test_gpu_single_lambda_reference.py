@@ -36,32 +36,22 @@ gamma_1 grad f(x_1)) is bounded componentwise (no contraction is assumed: gamma_
     |dx_2| <= 2 [B1 + gamma_1 dG(x_1) + |d gamma_1| |grad f(x_1)| + 2 u (|x_1| + gamma_1 |grad f(x_1)|) + (u gamma_1 + |d gamma_1|) lambda]
 
 The shapes come from a restatement of the work split of each kernel (api.cu: fused_cluster_size, fused_plan, plan_dense,
-solver_grid, gridres_eligible; gemv.cuh: csr_lanes_per_row, gsum_slice; solver_fused.cuh: fused_pass, fused_gradient_slice).
+solver_grid, gridres_eligible; gemv.cuh: csr_lanes_per_row, gsum_slice; solver_fused.cuh: fused_pass, fused_gradient_slice);
+the parts the primal-dual reference test shares live in tests/kernel_plan.py.
 A CPU test asserts that the shape set reaches every branch at 148 SMs, a GPU test at the device's SM count.  The CPU self-check
 shows that the bounds reject a result with one 2048-column chunk of A x, one row of A' r, one 8192-column CTA slice or one CSR
 non-zero left out, and accept a float64 evaluation in another summation order.
 """
-import contextlib
 import functools
-import os
 
 import numpy as np
 import pytest
-import scipy.sparse as sp
 
+from kernel_plan import DENSE_REQUIRED, _csr, cdiv, csr_branches, dense_branches, environ, r16
 from xprec_reference import LD, U, Term, reference, within, within_cols
 
 B200_SMEM_OPTIN = 232448          # cudaDevAttrMaxSharedMemoryPerBlockOptin of a B200 (227 KB)
-KCHUNK, KFCOLS, KFMAXC = 2048, 8192, 16
-SMALL_BYTES = 8 << 20             # api.cu: kSmallProblemBytes
-
-
-def r16(n):
-    return -(-n // 16) * 16
-
-
-def cdiv(a, b):
-    return -(-a // b)
+KFCOLS, KFMAXC = 8192, 16
 
 
 # ---------------------------------------------------------------- restatement of the kernel selection
@@ -119,81 +109,6 @@ FUSED_REQUIRED = {f"C:{c}" for c in range(1, 17)} | {"last:16", "last:8192", "n%
                                                       "rows<clusters", "helpers"}
 
 
-def plan_dense(m, n, grid):
-    """api.cu: plan_dense at upload, for the handle's grid (2 CTAs per SM) -> (nchunks, rb, nrb)."""
-    nch = cdiv(n, KCHUNK)
-    rb = 64
-    while rb > 8 and nch * cdiv(m, rb) < 16 * grid:
-        rb //= 2
-    return nch, rb, cdiv(m, rb)
-
-
-def solver_grid(m, n, sm, grid, env_grid=None):
-    """api.cu: solver_grid for a dense least-squares term (ADAPROX_GRID = env_grid)."""
-    if env_grid:
-        return min(env_grid, grid)
-    return min(grid, sm) if m * r16(n) * 8 < SMALL_BYTES else grid
-
-
-def dense_branches(shapes, sm):
-    grid = 2 * sm
-    hit = set()
-    for m, n, env_grid in shapes:
-        nch, rb, nrb = plan_dense(m, n, grid)
-        G = solver_grid(m, n, sm, grid, env_grid)
-        Uu = nch * nrb
-        hit.add(f"rb:{rb}")
-        hit.add("grid:env" if env_grid else ("grid:sm" if G == min(grid, sm) and G < grid else "grid:2sm"))
-        if env_grid and Uu % G:
-            hit.add("grid:env_nondiv")
-        if nch == 1:
-            hit.add("chunks:1")                      # phases.cuh: f_rows_local
-        elif nch <= 4 and r16(n) % KCHUNK:
-            hit.add("chunks:2-4_ragged")
-        bounds = [(Uu * b // G, Uu * (b + 1) // G) for b in range(G)]
-        if any(u0 == u1 for u0, u1 in bounds):
-            hit.add("idle_cta")
-        if any(u0 < u1 and u0 % nrb and (u1 - 1) // nrb > u0 // nrb for u0, u1 in bounds):
-            hit.add("slab_mid_chunk_crossing")
-        hit.add("gsum:warp" if (G > 16 * nch and nrb > 16) else "gsum:thread")    # gemv.cuh: gsum_slice
-        if m % 4:
-            hit.add("m%4")                           # gemv_t_dense: row remainder
-    return hit
-
-
-DENSE_REQUIRED = {"rb:8", "rb:16", "rb:32", "rb:64", "grid:sm", "grid:2sm", "grid:env", "grid:env_nondiv", "chunks:1",
-                  "chunks:2-4_ragged", "idle_cta", "slab_mid_chunk_crossing", "gsum:warp", "gsum:thread", "m%4"}
-
-
-def csr_lanes_per_row(nnz, nrows):
-    """gemv.cuh: csr_lanes_per_row"""
-    avg = nnz // max(nrows, 1)
-    return 32 if avg > 192 else (16 if avg > 24 else (8 if avg > 12 else 4))
-
-
-def csr_branches(cases):
-    hit = set()
-    for name, kind, lpr in cases:
-        X = CSR_MATRICES[name]()
-        m, nf = X.shape
-        how = "forced" if lpr else "mean"
-        ln = lpr or csr_lanes_per_row(X.nnz, m)
-        lt = lpr or csr_lanes_per_row(X.nnz, nf)
-        hit |= {f"Xw:{ln}:{how}", f"Xtr:{lt}:{how}", f"kind:{kind}"}
-        lens = set(np.diff(X.indptr).tolist())
-        if {0, 1, ln - 1, 4 * ln, 4 * ln + 1} <= lens and max(lens) > 2000:
-            hit.add(f"rows:{ln}")
-        if np.any(np.bincount(X.indices, minlength=nf) == 0):
-            hit.add("empty_feature")
-        if m < 32 // ln:
-            hit.add("rows<group")
-    return hit
-
-
-CSR_REQUIRED = ({f"{d}:{k}:{h}" for d in ("Xw", "Xtr") for k in (4, 8, 16, 32) for h in ("mean", "forced")} |
-                {f"rows:{k}" for k in (4, 8, 16, 32)} | {"kind:lsq", "kind:logistic", "empty_feature", "rows<group"})
-
-
 def gridres_x_in_smem(m, n, sm, optin=B200_SMEM_OPTIN):
     """api.cu: gridres_eligible -> True / False (x in shared / global memory); None: not eligible."""
     ld = r16(n)
@@ -211,6 +126,10 @@ def resident_fits(m, n, optin=B200_SMEM_OPTIN):
     return ld <= 1024 and 8 * (rows_cap * ld + 2 * ld + 2 * rows_cap + 16 + 32) + 1024 <= optin
 
 
+CSR_REQUIRED = ({f"{d}:{k}:{h}" for d in ("Xw", "Xtr") for k in (4, 8, 16, 32) for h in ("mean", "forced")} |
+                {f"rows:{k}" for k in (4, 8, 16, 32)} | {"kind:lsq", "kind:logistic", "empty_feature", "rows<group"})
+
+
 # ---------------------------------------------------------------- the shape sets
 # fused: (m, n, ADAPROX_FUSED_CHUNK, helpers); n = 8192 (C - 1) + w
 FUSED_CASES = [(3, 16, None, False), (70, 8192, "5", False), (45, 8192 + 16, "64", False), (100, 2 * 8192 + 4001, None, False),
@@ -224,19 +143,6 @@ DENSE_CASES = [(5, 40, None), (1000, 1000, None), (1003, 5000, None), (700, 4100
                (75777, 16, None), (151553, 16, None), (303105, 8, None), (2, 6000, None)]
 RESIDENT_CASES = [(400, 1000), (100, 300), (7, 1), (5, 1024), (33, 517), (416, 1024)]
 GRIDRES_CASES = [(500, 1000), (4000, 1000), (120, 40), (1, 1024), (3000, 517), (4100, 1024), (4144, 1000)]
-
-
-def _csr(m, nf, lengths, seed, empty=(1,)):
-    """CSR with the given row lengths (cycled, capped at the usable features); the features in `empty` have no non-zeros."""
-    rng = np.random.default_rng(seed)
-    pool = np.array([c for c in range(nf) if c not in empty])
-    indptr, cols = [0], []
-    for i in range(m):
-        k = min(lengths[i % len(lengths)], pool.size)
-        cols.append(np.sort(rng.choice(pool, size=k, replace=False)) if k else np.zeros(0, dtype=np.int64))
-        indptr.append(indptr[-1] + k)
-    ind = np.concatenate(cols).astype(np.int32)
-    return sp.csr_matrix((rng.uniform(-1.0, 1.0, ind.size), ind, np.array(indptr)), shape=(m, nf))
 
 
 MIXED_LENGTHS = [0, 1, 3, 7, 15, 31, 4, 16, 17, 8, 32, 33, 64, 65, 128, 129, 2100]
@@ -255,7 +161,7 @@ CSR_CASES = ([(name, kind, None) for name in CSR_MATRICES for kind in ("lsq", "l
 
 def _assert_reaches_everything(sm):
     for hit, req in ((fused_branches(FUSED_CASES, sm), FUSED_REQUIRED), (dense_branches(DENSE_CASES, sm), DENSE_REQUIRED),
-                     (csr_branches(CSR_CASES), CSR_REQUIRED)):
+                     (csr_branches(CSR_CASES, CSR_MATRICES), CSR_REQUIRED)):
         assert req <= hit, (sm, sorted(req - hit))
     xs = {gridres_x_in_smem(m, n, sm) for m, n in GRIDRES_CASES}
     assert xs == {True, False}, (sm, xs)
@@ -401,20 +307,6 @@ def test_bounds_reject_dropped_contributions_and_accept_another_order():
 
 
 # ---------------------------------------------------------------- device against the reference
-@contextlib.contextmanager
-def environ(env):
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update({k: str(v) for k, v in env.items()})
-    try:
-        yield
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-
-
 def _check(AdaProx, fd, term, k, seed, env, passes):
     x0, gam, lam, gam_our = _instance(term, k, seed)
     R = full_reference(term, x0, gam, lam, gam_our)
