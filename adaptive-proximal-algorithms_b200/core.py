@@ -850,6 +850,68 @@ def adaptive_proxgrad_path(X0=None, *, f, lambdas, rule, gamma0=None, tol=1e-5, 
     return np.ascontiguousarray(xoT.T), its, info
 
 
+def adaptive_primal_dual_path(X0=None, Y0=None, *, f, A, upper, rule, lower=0.0, gamma0=None, tol=1e-5, maxit=10_000, history=0):
+    """Batched C path of the dual SVM (dual_svm/runme.jl:47-59; include/adaprox.h: adaprox_solve_box_path): column j of
+    the result is what ``adaptive_primal_dual(X0[:, j], [Y0[j]], f=f, g=IndBox(lower, upper[j]), h=IndZero(), A=A,
+    rule=rule_j, tol=tol, maxit=maxit)`` returns, where rule_j is ``rule`` with ``gamma = gamma0[j]`` when ``gamma0`` is given
+    (condat_vu's parameters arrive as a ``FixedStepsize``).  ``f`` is a ``Quadratic`` or a ``QuadraticGram`` over a dense
+    matrix, ``A`` the 1 x n label row.  X0 (n, L) and Y0 (L,) default to zeros.  Returns ``(X, Y, its, info)`` with X of
+    shape (n, L), Y the L dual scalars, ``its`` the per-column iteration counts and ``info`` holding per-column
+    ``norm_res``, ``gamma``, ``sigma``, ``f_x`` and, with ``history = H > 0``, the arrays ``gamma_hist``, ``res_hist``,
+    ``obj_hist`` (objective f + g + h(A x)) of shape (min(H, maxit), L) (NaN after a column stopped)."""
+    ff, _ = _unwrap(f)
+    AA, _ = _unwrap(A)
+    if not isinstance(ff, _Smooth):
+        raise L.AdaproxError(-3, f"eval_with_pullback not defined for type {type(ff).__name__} (no CPU fallback)")
+    dev = ff._dev()
+    Amat = _as_matrix(AA, dev)
+    n = Amat.shape[1]
+    up = np.ascontiguousarray(np.asarray(upper, dtype=F64).ravel())
+    Lc = up.shape[0]
+    if np.ndim(upper) != 1 or Lc < 1:
+        raise ValueError("upper must be a non-empty vector of box bounds")
+    p = ff._problem(n)
+    p.g = IndBox(float(lower), float(lower))._desc()
+    p.h = IndZero()._desc()
+    p.A_mat, p.m_dual = Amat.id, Amat.shape[0]
+    o = _opts(tol, maxit)
+    rule._fill(o)
+    o.solver = L.S_ADAPTIVE_PRIMAL_DUAL
+    x0T = y0 = g0 = None
+    if X0 is not None:
+        X0 = np.asarray(X0, dtype=F64)
+        if X0.shape != (n, Lc):
+            raise ValueError(f"X0 has shape {X0.shape}, expected {(n, Lc)}")
+        x0T = np.ascontiguousarray(X0.T)
+    if Y0 is not None:
+        y0 = np.ascontiguousarray(np.asarray(Y0, dtype=F64))
+        if y0.shape != (Lc,):
+            raise ValueError(f"Y0 has shape {y0.shape}, expected {(Lc,)}")
+    if gamma0 is not None:
+        g0 = np.ascontiguousarray(np.asarray(gamma0, dtype=F64))
+        if g0.shape != (Lc,):
+            raise ValueError("gamma0 must have one entry per C value")
+    xoT = np.empty((Lc, n), dtype=F64)
+    yo = np.empty(Lc, dtype=F64)
+    its = np.zeros(Lc, dtype=np.int64)
+    nres, gout, sout, fout = (np.empty(Lc, dtype=F64) for _ in range(4))
+    H = int(min(history, maxit)) if history else 0
+    hist = np.empty((3, max(H, 1), Lc), dtype=F64) if H > 0 else None
+    res = L.Result()
+    opt = lambda a: _dp(a) if a is not None else None
+    dev.check(dev.lib.adaprox_solve_box_path(dev.h, C.byref(p), C.byref(o), Lc, _dp(up), opt(g0), opt(x0T), opt(y0), _dp(xoT), _dp(yo),
+                                             its.ctypes.data_as(C.POINTER(C.c_int64)), _dp(nres), _dp(gout), _dp(sout), _dp(fout),
+                                             opt(hist), H, C.byref(res)))
+    dev.launches += res.kernel_launches
+    info = dict(norm_res=nres, gamma=gout, sigma=sout, f_x=fout, flags=int(res.flags), solve_ms=res.solve_ms,
+                kernel_launches=int(res.kernel_launches), batched_evals=int(res.f_evals), iters_max=int(res.iters))
+    if hist is not None:
+        info.update(gamma_hist=hist[0], res_hist=hist[1], obj_hist=hist[2])
+    _last_info.update(dict(flags=info["flags"], solve_ms=res.solve_ms, kernel_launches=int(res.kernel_launches),
+                           matrix_passes=int(res.matrix_passes)))
+    return np.ascontiguousarray(xoT.T), yo, its, info
+
+
 def auto_adaptive_proxgrad(x, *, f, g, gamma=None, tol=1e-5, maxit=100_000, name="AutoAdaPGM", log=None):
     """src/AdaProx.jl:423-455: two gradient evaluations and one (or two) prox steps estimate the initial stepsize, then
     AdaPGM with OurRule from the ORIGINAL point.  Every oracle call below is a device call (eval_with_gradient / prox

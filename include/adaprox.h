@@ -245,6 +245,29 @@ int adaprox_solve_lambda_path(adaprox_handle h, const adaprox_problem* p, const 
                               const double* lambdas, const double* gamma0, const double* x0T, double* x_outT,
                               int64_t* iters, double* norm_res, double* gamma_out, double* f_out,
                               double* hist, int64_t hist_rows, adaprox_result* res);
+/* ---- batched C path of the dual SVM (dual_svm/runme.jl:47-59) ------------------ */
+/* AdaPDM (src/AdaProx.jl:312-364; Condat-Vu :367-416 through RULE_FIXED) on the L problems
+ *     min_x f(x) + IndBox(lower, upper[j])(x) + IndZero(A x) ,  j = 0 .. L-1
+ * that share f, the lower bound and the one-row linear map A of `p`:
+ *   - f (p->f_kind) is a dense QUADRATIC (Q, q) or a dense QUADRATIC_GRAM (Z, q); a row-sharded matrix is refused (split
+ *     the C values over the ranks instead);
+ *   - p->g is an IndBox with scalar bounds: p->g.lo is the common lower bound, p->g.hi is ignored;
+ *   - p->h is IndZero and p->A_mat a dense 1 x n matrix (the labels y');
+ *   - o->solver is ADAPROX_S_ADAPTIVE_PRIMAL_DUAL with any of the four rules.
+ * Anything else returns ADAPROX_ERR_UNSUPPORTED; upper[j] < lower, a NaN upper[j] or L < 1 return ADAPROX_ERR_INVALID.
+ * Column j is what adaprox_solve returns for the single problem with g = IndBox(lower, upper[j]), x0 = x0T[j], y0 = y0[j]
+ * and, when gamma0 is given, o->gamma = gamma0[j]: every column has its own stepsize state, dual scalar, residual and
+ * stopping iteration, and is frozen when it converges.  maxit = 0 returns x_1 and y_0 with iters 0.  The L iterates
+ * advance together: Q X (or Z (Z' X)) is an fp64 tensor-core contraction (mma.sync DMMA), the rest is one CTA per column.
+ *   upper   : [L] box bounds C_j;  gamma0 : [L] initial (FixedStepsize: fixed) stepsizes, or NULL for o->gamma
+ *   x0T     : [L][n] (column j contiguous), or NULL for zeros;  y0 : [L] initial dual scalars, or NULL for zeros
+ *   x_outT  : [L][n];  y_out / iters / norm_res / gamma_out / sigma_out / f_out : [L] (each may be NULL)
+ *   hist    : optional 3 * hist_rows * L doubles: gamma, norm_res, objective f + g + h(A x) per (iteration - 1, column);
+ *             NaN where a column had already stopped.  res->iters = largest per-column iteration count. */
+int adaprox_solve_box_path(adaprox_handle h, const adaprox_problem* p, const adaprox_options* o, int64_t L,
+                           const double* upper, const double* gamma0, const double* x0T, const double* y0,
+                           double* x_outT, double* y_out, int64_t* iters, double* norm_res, double* gamma_out,
+                           double* sigma_out, double* f_out, double* hist, int64_t hist_rows, adaprox_result* res);
 /* which: 0 = R = A X - b (K = n), 1 = G = A' R (K = m); mean device ms per launch over `reps` launches on an L-column
  * batch of zeros (measurement hook of tools/bench_configs.py) */
 int adaprox_time_path_gemm(adaprox_handle h, adaprox_id mat, int64_t L, int which, int reps, double* ms_per_launch);

@@ -295,6 +295,34 @@ function adaptive_proxgrad_path(X0::Union{Nothing,Matrix{Float64}}; f, lambdas::
     return X, its, (norm_res = nres, gamma = gam, f_x = fx, solve_ms = res.solve_ms)
 end
 
+# ---- batched C path of the dual SVM (include/adaprox.h: adaprox_solve_box_path) ----------------------------------
+# Column j of the result is what `adaptive_primal_dual(X0[:, j], [Y0[j]]; f, g = IndBox(lower, upper[j]), h = IndZero(), A,
+# rule, tol, maxit)` returns; f is Quadratic(Q, q) or QuadraticGram(Z, q), A the 1 x n label row.  NOT EXECUTED (no Julia
+# in the build image).
+function adaptive_primal_dual_path(X0::Union{Nothing,Matrix{Float64}}, Y0::Union{Nothing,Vector{Float64}}; f, A,
+                                   upper::Vector{Float64}, rule, lower = 0.0, gamma0 = nothing, tol = 1e-5, maxit = 10_000)
+    L = length(upper)
+    fo = device_oracle(unwrap(f))
+    n = size(unwrap(A), 2)
+    prob = CProblem(fo.kind, fo.ipar, fo.mat, fo.vec, fo.c, CProx(4, 0, 1.0, Float64(lower), Float64(lower), 0, 0, 0),
+                    device_prox(ProximalCore.IndZero()), upload(unwrap(A)), n, 1)
+    o = options(0; rule = rule_fields(rule), tol, maxit, want = Int32(0), counting = cflags(f, nothing, nothing, A))
+    X = Matrix{Float64}(undef, n, L)                          # column-major: column j contiguous = the library's [L][n] layout
+    Y = zeros(L); its = zeros(Int64, L); nres = zeros(L); gam = zeros(L); sig = zeros(L); fx = zeros(L)
+    res = CResult()
+    x0ptr = X0 === nothing ? Ptr{Float64}(C_NULL) : pointer(X0)
+    y0ptr = Y0 === nothing ? Ptr{Float64}(C_NULL) : pointer(Y0)
+    g0ptr = gamma0 === nothing ? Ptr{Float64}(C_NULL) : pointer(gamma0)
+    GC.@preserve X0 Y0 gamma0 upper X Y its nres gam sig fx begin
+        check(ccall((:adaprox_solve_box_path, lib), Cint,
+                    (Handle, Ref{CProblem}, Ref{COptions}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                     Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                     Ptr{Float64}, Int64, Ref{CResult}),
+                    handle(), prob, o, L, upper, g0ptr, x0ptr, y0ptr, X, Y, its, nres, gam, sig, fx, C_NULL, 0, res))
+    end
+    return X, Y, its, (norm_res = nres, gamma = gam, sigma = sig, f_x = fx, solve_ms = res.solve_ms)
+end
+
 # ---- multi-GPU: peer exchange blocks for the all-reduce inside the kernels (adaprox_p2p_*) -----------------------
 # `allgather` is supplied by the caller (e.g. MPI.Allgather on the 64-byte handles); rank order.  NOT EXECUTED.
 function attach_p2p(n_max::Integer, nranks::Integer, rank::Integer, allgather::Function)
