@@ -15,7 +15,7 @@ from .core import (                                               # noqa: F401
     Zero, IndZero, NormL1, NormL2, IndBox, Translate, convex_conjugate, prox,
     eval_with_pullback, eval_with_gradient,
     FixedStepsize, MalitskyMishchenkoRule, OurRule, OurRulePlus, stepsize,
-    adaptive_primal_dual, adaptive_primal_dual_path, condat_vu, adaptive_proxgrad, auto_adaptive_proxgrad, adaptive_proxgrad_path, fixed_proxgrad, adaptive_linesearch_primal_dual, malitsky_pock,
+    adaptive_primal_dual, adaptive_primal_dual_path, adaptive_primal_dual_lambda_path, condat_vu, adaptive_proxgrad, auto_adaptive_proxgrad, adaptive_proxgrad_path, fixed_proxgrad, adaptive_linesearch_primal_dual, malitsky_pock,
     backtracking_proxgrad, backtracking_nesterov, fixed_nesterov, agraal,
     generate_planted_lasso, last_solve_info,
 )

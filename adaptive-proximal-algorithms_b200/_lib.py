@@ -93,6 +93,8 @@ SYMBOLS = {
                                             C.POINTER(C.c_int64), c_dp, c_dp, c_dp, c_dp, C.c_int64, C.POINTER(Result)]),
     "adaprox_solve_box_path": (C.c_int, [_h, C.POINTER(Problem), C.POINTER(Options), C.c_int64, c_dp, c_dp, c_dp, c_dp, c_dp, c_dp,
                                          C.POINTER(C.c_int64), c_dp, c_dp, c_dp, c_dp, c_dp, C.c_int64, C.POINTER(Result)]),
+    "adaprox_solve_pd_lambda_path": (C.c_int, [_h, C.POINTER(Problem), C.POINTER(Options), C.c_int64, c_dp, c_dp, c_dp, c_dp, c_dp,
+                                               c_dp, C.POINTER(C.c_int64), c_dp, c_dp, c_dp, c_dp, C.c_int64, C.POINTER(Result)]),
     "adaprox_time_path_gemm":(C.c_int, [_h, c_id, C.c_int64, C.c_int, C.c_int, c_dp]),
     "adaprox_comm_unique_id": (C.c_int, [C.c_void_p]),
     "adaprox_comm_init": (C.c_int, [_h, C.c_int, C.c_int, C.c_void_p]),

@@ -912,6 +912,71 @@ def adaptive_primal_dual_path(X0=None, Y0=None, *, f, A, upper, rule, lower=0.0,
     return np.ascontiguousarray(xoT.T), yo, its, info
 
 
+def adaptive_primal_dual_lambda_path(X0=None, Y0=None, *, f, h, A, lambdas, rule, gamma0=None, tol=1e-5, maxit=10_000, history=0):
+    """Batched lambda path of LAD and the square-root lasso (least_absolute_deviation/runme.jl, square_root_lasso/runme.jl;
+    include/adaprox.h: adaprox_solve_pd_lambda_path): column j of the result is what ``adaptive_primal_dual(X0[:, j],
+    Y0[:, j], f=f, g=NormL1(lambdas[j]), h=h, A=A, rule=rule_j, tol=tol, maxit=maxit)`` returns, where rule_j is ``rule``
+    with ``gamma = gamma0[j]`` when ``gamma0`` is given (condat_vu's parameters arrive as a ``FixedStepsize``).  ``f`` is
+    ``Zero()``, ``h`` a ``NormL1`` / ``NormL2`` of any weight, optionally ``Translate``'d, and ``A`` a dense m x n matrix.
+    X0 (n, L) and Y0 (m, L) default to zeros.  Returns ``(X, Y, its, info)`` with X of shape (n, L), Y of shape (m, L),
+    ``its`` the per-column iteration counts and ``info`` holding per-column ``norm_res``, ``gamma``, ``sigma`` and, with
+    ``history = H > 0``, the arrays ``gamma_hist``, ``res_hist``, ``obj_hist`` (objective g + h(A x)) of shape
+    (min(H, maxit), L) (NaN after a column stopped)."""
+    ff, _ = _unwrap(f)
+    hh, _ = _unwrap(h)
+    AA, _ = _unwrap(A)
+    if not isinstance(ff, _Smooth):
+        raise L.AdaproxError(-3, f"eval_with_pullback not defined for type {type(ff).__name__} (no CPU fallback)")
+    dev = ff._dev()
+    Amat = _as_matrix(AA, dev)
+    m, n = Amat.shape
+    if np.ndim(lambdas) != 1 or np.size(lambdas) < 1:
+        raise ValueError("lambdas must be a non-empty vector")
+    lam = np.ascontiguousarray(np.asarray(lambdas, dtype=F64))
+    Lc = lam.shape[0]
+    p = ff._problem(n)
+    p.g = NormL1(1.0)._desc()
+    p.h = hh._desc()
+    p.A_mat, p.m_dual = Amat.id, m
+    o = _opts(tol, maxit)
+    rule._fill(o)
+    o.solver = L.S_ADAPTIVE_PRIMAL_DUAL
+    x0T = y0T = g0 = None
+    if X0 is not None:
+        X0 = np.asarray(X0, dtype=F64)
+        if X0.shape != (n, Lc):
+            raise ValueError(f"X0 has shape {X0.shape}, expected {(n, Lc)}")
+        x0T = np.ascontiguousarray(X0.T)
+    if Y0 is not None:
+        Y0 = np.asarray(Y0, dtype=F64)
+        if Y0.shape != (m, Lc):
+            raise ValueError(f"Y0 has shape {Y0.shape}, expected {(m, Lc)}")
+        y0T = np.ascontiguousarray(Y0.T)
+    if gamma0 is not None:
+        g0 = np.ascontiguousarray(np.asarray(gamma0, dtype=F64))
+        if g0.shape != (Lc,):
+            raise ValueError("gamma0 must have one entry per lambda")
+    xoT = np.empty((Lc, n), dtype=F64)
+    yoT = np.empty((Lc, m), dtype=F64)
+    its = np.zeros(Lc, dtype=np.int64)
+    nres, gout, sout = (np.empty(Lc, dtype=F64) for _ in range(3))
+    H = int(min(history, maxit)) if history else 0
+    hist = np.empty((3, max(H, 1), Lc), dtype=F64) if H > 0 else None
+    res = L.Result()
+    opt = lambda a: _dp(a) if a is not None else None
+    dev.check(dev.lib.adaprox_solve_pd_lambda_path(dev.h, C.byref(p), C.byref(o), Lc, _dp(lam), opt(g0), opt(x0T), opt(y0T), _dp(xoT),
+                                                   _dp(yoT), its.ctypes.data_as(C.POINTER(C.c_int64)), _dp(nres), _dp(gout), _dp(sout),
+                                                   opt(hist), H, C.byref(res)))
+    dev.launches += res.kernel_launches
+    info = dict(norm_res=nres, gamma=gout, sigma=sout, flags=int(res.flags), solve_ms=res.solve_ms,
+                kernel_launches=int(res.kernel_launches), batched_evals=int(res.f_evals), iters_max=int(res.iters))
+    if hist is not None:
+        info.update(gamma_hist=hist[0], res_hist=hist[1], obj_hist=hist[2])
+    _last_info.update(dict(flags=info["flags"], solve_ms=res.solve_ms, kernel_launches=int(res.kernel_launches),
+                           matrix_passes=int(res.matrix_passes)))
+    return np.ascontiguousarray(xoT.T), np.ascontiguousarray(yoT.T), its, info
+
+
 def auto_adaptive_proxgrad(x, *, f, g, gamma=None, tol=1e-5, maxit=100_000, name="AutoAdaPGM", log=None):
     """src/AdaProx.jl:423-455: two gradient evaluations and one (or two) prox steps estimate the initial stepsize, then
     AdaPGM with OurRule from the ORIGINAL point.  Every oracle call below is a device call (eval_with_gradient / prox

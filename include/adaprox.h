@@ -268,6 +268,30 @@ int adaprox_solve_box_path(adaprox_handle h, const adaprox_problem* p, const ada
                            const double* upper, const double* gamma0, const double* x0T, const double* y0,
                            double* x_outT, double* y_out, int64_t* iters, double* norm_res, double* gamma_out,
                            double* sigma_out, double* f_out, double* hist, int64_t hist_rows, adaprox_result* res);
+/* ---- batched lambda path of LAD and the square-root lasso (least_absolute_deviation/runme.jl, square_root_lasso/runme.jl) */
+/* AdaPDM (src/AdaProx.jl:312-364; Condat-Vu :367-416 through RULE_FIXED) on the L problems
+ *     min_x lambdas[j] |x|_1 + h(A x) ,  j = 0 .. L-1
+ * that share h and the m x n linear map A of `p`:
+ *   - p->f_kind is ZERO;
+ *   - p->g is a NormL1 (no shift, not conjugated); its weight is replaced by lambdas[j];
+ *   - p->h is a NormL1 or a NormL2 of any weight, optionally with a shift (Translate(NormL1(), -b) is LAD,
+ *     Translate(NormL2(), -b) the square-root lasso), not conjugated;
+ *   - p->A_mat is a dense matrix; a row-sharded A is refused (split the lambda values over the ranks instead);
+ *   - o->solver is ADAPROX_S_ADAPTIVE_PRIMAL_DUAL with any of the four rules (AdaPDM+ is refused).
+ * Anything else returns ADAPROX_ERR_UNSUPPORTED; a negative or NaN lambda or L < 1 return ADAPROX_ERR_INVALID.
+ * Column j is what adaprox_solve returns for the single problem with g = NormL1(lambdas[j]), x0 = x0T[j], y0 = y0T[j] and,
+ * when gamma0 is given, o->gamma = gamma0[j]: every column has its own stepsize state, dual vector, residual and stopping
+ * iteration, and is frozen when it converges.  maxit = 0 returns x_1 and y_0 with iters 0.  The L iterates advance
+ * together: A X and A' Y are fp64 tensor-core contractions (mma.sync DMMA), the rest is one CTA per column.
+ *   gamma0  : [L] initial (FixedStepsize: fixed) stepsizes, or NULL for o->gamma
+ *   x0T     : [L][n], y0T : [L][m] (column j contiguous), or NULL for zeros
+ *   x_outT  : [L][n];  y_outT : [L][m] or NULL;  iters / norm_res / gamma_out / sigma_out : [L] (each may be NULL)
+ *   hist    : optional 3 * hist_rows * L doubles: gamma, norm_res, objective g + h(A x) per (iteration - 1, column);
+ *             NaN where a column had already stopped.  res->iters = largest per-column iteration count. */
+int adaprox_solve_pd_lambda_path(adaprox_handle h, const adaprox_problem* p, const adaprox_options* o, int64_t L,
+                                 const double* lambdas, const double* gamma0, const double* x0T, const double* y0T,
+                                 double* x_outT, double* y_outT, int64_t* iters, double* norm_res, double* gamma_out,
+                                 double* sigma_out, double* hist, int64_t hist_rows, adaprox_result* res);
 /* which: 0 = R = A X - b (K = n), 1 = G = A' R (K = m); mean device ms per launch over `reps` launches on an L-column
  * batch of zeros (measurement hook of tools/bench_configs.py) */
 int adaprox_time_path_gemm(adaprox_handle h, adaprox_id mat, int64_t L, int which, int reps, double* ms_per_launch);

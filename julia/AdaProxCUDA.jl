@@ -323,6 +323,33 @@ function adaptive_primal_dual_path(X0::Union{Nothing,Matrix{Float64}}, Y0::Union
     return X, Y, its, (norm_res = nres, gamma = gam, sigma = sig, f_x = fx, solve_ms = res.solve_ms)
 end
 
+# ---- batched lambda path of LAD and the square-root lasso (include/adaprox.h: adaprox_solve_pd_lambda_path) --------
+# Column j of the result is what `adaptive_primal_dual(X0[:, j], Y0[:, j]; f = Zero(), g = NormL1(lambdas[j]), h, A, rule,
+# tol, maxit)` returns; h is NormL1 / NormL2, optionally Translate'd, A a dense matrix.  NOT EXECUTED (no Julia in the
+# build image).
+function adaptive_primal_dual_lambda_path(X0::Union{Nothing,Matrix{Float64}}, Y0::Union{Nothing,Matrix{Float64}}; h, A,
+                                          lambdas::Vector{Float64}, rule, gamma0 = nothing, tol = 1e-5, maxit = 10_000)
+    L = length(lambdas)
+    m, n = size(unwrap(A))
+    prob = CProblem(0, 0, 0, 0, 0.0, CProx(2, 0, 1.0, 0.0, 0.0, 0, 0, 0), device_prox(unwrap(h)), upload(unwrap(A)), n, m)
+    o = options(0; rule = rule_fields(rule), tol, maxit, want = Int32(0), counting = cflags(nothing, nothing, h, A))
+    X = Matrix{Float64}(undef, n, L)                          # column-major: column j contiguous = the library's [L][n] layout
+    Y = Matrix{Float64}(undef, m, L)
+    its = zeros(Int64, L); nres = zeros(L); gam = zeros(L); sig = zeros(L)
+    res = CResult()
+    x0ptr = X0 === nothing ? Ptr{Float64}(C_NULL) : pointer(X0)
+    y0ptr = Y0 === nothing ? Ptr{Float64}(C_NULL) : pointer(Y0)
+    g0ptr = gamma0 === nothing ? Ptr{Float64}(C_NULL) : pointer(gamma0)
+    GC.@preserve X0 Y0 gamma0 lambdas X Y its nres gam sig begin
+        check(ccall((:adaprox_solve_pd_lambda_path, lib), Cint,
+                    (Handle, Ref{CProblem}, Ref{COptions}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                     Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                     Ptr{Float64}, Int64, Ref{CResult}),
+                    handle(), prob, o, L, lambdas, g0ptr, x0ptr, y0ptr, X, Y, its, nres, gam, sig, C_NULL, 0, res))
+    end
+    return X, Y, its, (norm_res = nres, gamma = gam, sigma = sig, solve_ms = res.solve_ms)
+end
+
 # ---- multi-GPU: peer exchange blocks for the all-reduce inside the kernels (adaprox_p2p_*) -----------------------
 # `allgather` is supplied by the caller (e.g. MPI.Allgather on the 64-byte handles); rank order.  NOT EXECUTED.
 function attach_p2p(n_max::Integer, nranks::Integer, rank::Integer, allgather::Function)
